@@ -11,13 +11,19 @@ batch.
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config clevr|shapes|vqa514|vqa2050|stress]
     python bench.py --impl reference ...        # CPU arm (the oracle restatement of the reference)
 
-How the number is taken (VERDICT r1: a 20-step region is ~1 ms of host wake-up noise): the block of
-K steps is repeated R times back to back, R chosen from a calibration run so that one timed region
-lasts >= --min-seconds (0.5 s), each region bracketed by barrier + synchronize and timed with CUDA
-events; `--trials` (3) regions are taken and the MEDIAN is reported (`repeats`, `timed_region_s`,
-`trial_values` are in the line). Under torchrun every rank owns one GPU and its own shard of the
-questions (weak scaling, no data-path collective: questions are independent, SURVEY.md §8e);
-region time = max over ranks; rank 0 prints ONE JSON line.
+How the number is taken: --warmup W steps, then exactly --steps K timed steps, queued back to back
+on the executor pool and walking the resident batches round-robin. The warm-up is queued right
+before the timed steps, so the pool's worker threads and streams are already running when the
+timed steps begin; CUDA events on the current stream bracket the K timed steps only. A step takes
+~10 us on a B200 (1000 W power limit), so K in the thousands keeps the fill and drain of the pool's
+streams and host noise out of the number (measured there with W=20: 5.6-5.8 M questions/s at
+K=200, 6.4 M at K=4000). Under torchrun every rank owns one GPU and its own shard of the questions
+(weak scaling, no data-path collective: questions are independent, SURVEY.md §8e); region time =
+max over ranks; rank 0 prints ONE JSON line.
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0's shard) as DIR/scores.npy
+(float32 [B, C]) and DIR/validity.npy (float32 [B], 1 = the layout assembled). Inputs, weights and
+layouts are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -67,15 +73,17 @@ L2_BYTES = 126e6
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
-    ap.add_argument('--warmup', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=200, help='timed steps')
+    ap.add_argument('--warmup', type=int, default=20, help='untimed steps before them')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the last timed step\'s scores / validity to DIR/<name>.npy')
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--config', default='clevr', choices=sorted(WORKLOADS))
     ap.add_argument('--batch', type=int, default=0, help='questions per GPU per step (0 = the config\'s)')
     ap.add_argument('--layouts', default=None, choices=['expert', 'random', 'deep'],
                     help='CLEVR layout set (default expert)')
-    ap.add_argument('--min-seconds', type=float, default=0.5, help='length of one timed region')
-    ap.add_argument('--trials', type=int, default=3, help='timed regions; the median is reported')
+    ap.add_argument('--min-seconds', type=float, default=0.5, help='ignored (old command lines)')
+    ap.add_argument('--trials', type=int, default=3, help='ignored (old command lines)')
     ap.add_argument('--cpu-seconds', type=float, default=10.0, help='cpu_baseline sample budget')
     ap.add_argument('--ref-seconds', type=float, default=0.0,
                     help='--impl reference: stop after this many seconds (0 = run all --steps)')
@@ -97,7 +105,10 @@ def parse_args():
                     help='contexts/streams/worker threads (0 = the library default)')
     ap.add_argument('--host-threads', type=int, default=0, help='ignored (old command lines)')
     ap.add_argument('--pool', type=int, default=0, help='ignored (old command lines)')
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    return args
 
 
 def peaks():
@@ -328,7 +339,7 @@ def run_reference_arm(args, rank, world):
     port, ports_ms = best_cpu_port(wl, feat, word_vecs, weights, toks)
     for i in range(max(args.warmup, 1)):
         port.step(toks[i % 4])
-    steps = min(args.steps, 200)
+    steps = args.steps
     per = []
     t0 = time.perf_counter()
     for i in range(steps):
@@ -506,19 +517,52 @@ class Bench:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return float(t.item())
 
+    def block(self, first, n, toks=None, outs=None):
+        """Pre-marshalled steps first .. first+n-1 of the round-robin walk over the resident
+        batches; score buffers from the ring `self.outs` unless `outs` is given."""
+        toks = toks or self.toks
+        idx = [(first + j) % self.P for j in range(n)]
+        outs = outs or [self.outs[(first + j) % self.nout] for j in range(n)]
+        return self.pool.make_block([self.feats[i] for i in idx], [self.wvs[i] for i in idx],
+                                    [toks[i % len(toks)] for i in idx], outs)
+
     def blocks(self, steps, toks=None):
         """Pre-marshalled blocks of `steps` steps that together walk all P resident batches."""
-        P = self.P
-        nb = min(64, P // math.gcd(steps, P))
-        out = []
-        for b in range(nb):
-            idx = [(b * steps + j) % P for j in range(steps)]
-            tk = [(toks or self.toks)[i % len(toks or self.toks)] for i in idx]
-            out.append(self.pool.make_block([self.feats[i] for i in idx],
-                                            [self.wvs[i] for i in idx], tk,
-                                            [self.outs[(b * steps + j) % self.nout]
-                                             for j in range(steps)]))
-        return out
+        nb = min(64, self.P // math.gcd(steps, self.P))
+        return [self.block(b * steps, steps, toks) for b in range(nb)]
+
+    def headline(self, steps, warmup):
+        """`warmup` steps, then exactly `steps` timed steps. The warm-up is queued right before
+        the timed steps, so the timed steps start with the pool's worker threads running; CUDA
+        events bracket the timed steps only. Returns the timing and what the last timed step
+        computed: scores [B, C] float32 and validity bool[B]. That step writes a buffer of its
+        own: the ring `self.outs` is shared by steps of one launch group."""
+        torch = self.torch
+        last = torch.empty((self.B, self.wl['C']), dtype=torch.float32, device=self.dev)
+        outs = [self.outs[(warmup + j) % self.nout] for j in range(steps - 1)] + [last]
+        blk = self.block(warmup, steps, outs=outs)
+        warm = self.block(0, warmup) if warmup > 0 else None
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        self.barrier()
+        if warm is not None:
+            self.pool.begin()
+            self.pool.submit_block(warm)
+            self.pool.end()
+        l0 = self.pool.launch_count()
+        e0.record()
+        t0 = time.perf_counter()
+        self.pool.begin()
+        valid = self.pool.submit_block(blk)
+        self.pool.end()
+        e1.record()
+        host_ms = (time.perf_counter() - t0) * 1e3
+        self.barrier()
+        ms = self.allmax(e0.elapsed_time(e1))
+        return {'ms_per_step': ms / steps, 'timed_steps': steps,
+                'gpu_launches': self.pool.launch_count() - l0, 'timed_region_s': ms * 1e-3,
+                'host_enqueue_ms_per_step': host_ms / steps,
+                'value': self.world * self.B * steps / (ms * 1e-3),
+                'scores': last.cpu().numpy(), 'validity': valid[steps - 1].astype(bool)}
 
     def region(self, blocks, repeats):
         """`repeats` back-to-back repetitions of the step block, CUDA events on the current stream
@@ -781,13 +825,17 @@ def main():
     pool, ex, K = bn.pool, bn.ex, bn.K
     pk = peaks()
 
-    # ---- headline: device-resident inputs, median of `trials` regions of >= min_seconds
+    # ---- headline: device-resident inputs, --warmup steps then exactly --steps timed steps
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    head = bn.timed(args.steps, args.warmup, args.min_seconds, args.trials)
+    head = bn.headline(args.steps, args.warmup)
     launches = head['gpu_launches']
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name in ('scores', 'validity'):
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), head[name].astype(np.float32))
 
     # ---- the other two layout sets of SURVEY.md §8(d) (CLEVR: random valid; deep), same pool
     other_sets = None
@@ -930,9 +978,7 @@ def main():
             'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': head['ms_per_step'],
             'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
             'dtype': 'tf32 (fp32 in/out, fp32 accumulate)', 'data': 'synthetic',
-            'repeats': head['repeats'], 'timed_steps': head['timed_steps'],
-            'timed_region_s': head['timed_region_s'], 'trials': args.trials,
-            'trial_values': head['trial_values'],
+            'timed_steps': head['timed_steps'], 'timed_region_s': head['timed_region_s'],
             'config': dict({'workload': workload_title(wl, layouts), 'global_batch': B * world,
                             'parallelism': 'dp%d (question shards, no collective)' % world,
                             'cache': cache_note(bn),

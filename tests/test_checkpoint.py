@@ -2,6 +2,7 @@
 The file format is restated from its specification (TensorFlow cannot be installed here), so these
 tests pin the pieces that have known answers — CRC-32C test vector, LevelDB mask, block / footer
 layout byte by byte on a tiny table — and the round trip, including a Snappy-compressed block."""
+import os
 import struct
 
 import numpy as np
@@ -64,25 +65,28 @@ def test_snappy_blocks_and_prefix_compression():
     assert blk[0:3] == bytes([0, 11, 1]) and blk[15:18] == bytes([11, 5, 2])   # shared prefix 11
 
 
-def test_snappy_decoder_against_an_independent_encoder():
-    """TensorFlow compresses index blocks with Snappy: the decoder here against streams written by
-    the Snappy library itself (through pyarrow's codec) — variable-name-like text with long runs
-    (overlapping copies), > 60-byte literals (multi-byte literal lengths), random bytes, empty."""
-    pa = pytest.importorskip('pyarrow')
-    if not pa.Codec.is_available('snappy'):
-        pytest.skip('pyarrow without snappy')
-    codec = pa.Codec('snappy')
+def snappy_cases():
+    """Inputs of the Snappy streams in tests/golden/golden_snappy.npz (make_golden_snappy.py)."""
     rng = np.random.RandomState(0)
     names = [('neural_module_network/layout_execution/module_variables/%s/%s/%s%s' % (m, l, k, a))
              .encode() for m in ('FindModule', 'TransformModule', 'DescribeModule')
              for l in ('conv_image', 'fc_text', 'fc_att') for k in ('weights', 'biases')
              for a in ('', '/Adam', '/Adam_1')]
-    cases = [b'', b'a', b'ab' * 5000, b''.join(names), bytes(rng.randint(0, 256, 70000, dtype=np.uint8)),
-             b'\x00' * 100000, b''.join(names) * 40 + bytes(rng.randint(0, 4, 3000, dtype=np.uint8))]
-    for raw in cases:
-        comp = codec.compress(raw, asbytes=True)
-        assert ck._snappy_decompress(comp) == raw
-    assert len(codec.compress(cases[2], asbytes=True)) < 600      # it really compressed
+    return [b'', b'a', b'ab' * 5000, b''.join(names), bytes(rng.randint(0, 256, 70000, dtype=np.uint8)),
+            b'\x00' * 100000, b''.join(names) * 40 + bytes(rng.randint(0, 4, 3000, dtype=np.uint8))]
+
+
+def test_snappy_decoder_against_an_independent_encoder():
+    """TensorFlow compresses index blocks with Snappy: the decoder here against streams written by
+    the Snappy library itself (through pyarrow's codec, stored in tests/golden/golden_snappy.npz) —
+    variable-name-like text with long runs (overlapping copies), > 60-byte literals (multi-byte
+    literal lengths), random bytes, empty."""
+    z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'golden_snappy.npz'))
+    cases = snappy_cases()
+    assert len(z.files) == len(cases)
+    for i, raw in enumerate(cases):
+        assert ck._snappy_decompress(z['case_%d' % i].tobytes()) == raw
+    assert len(z['case_2']) < 600                                  # it really compressed
 
 
 def test_import_export_module_weights(tmp_path):
